@@ -18,7 +18,10 @@ every parameter and buffer written to HBM once.  Recording (Python module constr
            16-byte seed/offset broadcast (torchdistx_b200.parallel.sync_rng), once per step inside
            the e2e timed region; there is none in or between the kernels.
   --impl reference : the reference's own CPU materialize (oracle/_ref = pytorch/torchdistx
-           compiled from /root/reference) on a bounded sample of the same model, on the host cores.
+           compiled from the reference's sources) on a bounded sample of the same model, on the host cores.
+  --dump-outputs DIR : after the timed steps, every parameter and buffer of the model the `value`
+           steps wrote, as DIR/<name>.npy (see dump_outputs), for comparing two builds output for
+           output: the model, the seed and the step counts fix every value.
 """
 from __future__ import annotations
 
@@ -32,6 +35,7 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
@@ -239,9 +243,45 @@ class Ctx:
     """What every measurement of one run shares."""
 
 
-def measure_model(cx, model: str, steps: int, warmup: int, first_call: bool = False, roofline_only: bool = False):
+DUMP_BYTES = 60 << 20  # the arrays of --dump-outputs, in all (+ .npy headers and manifest.json: < 64 MB)
+
+
+def dump_outputs(model, out_dir: str):
+    """Writes each parameter and buffer of `model` as out_dir/<name>.npy -- float32 (exact for 16- and
+    32-bit floats) or float64 (float64 and integer tensors) -- and out_dir/manifest.json.  Tensors share
+    DUMP_BYTES, the smallest first; one that does not fit whole is written as the elements at the sorted
+    flat indices numpy.random.default_rng(zlib.crc32(name)).choice(numel, size=k, replace=False)."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    tensors = sorted(dict(list(model.named_parameters()) + list(model.named_buffers())).items(),
+                     key=lambda kv: kv[1].numel())
+    left, manifest = DUMP_BYTES, {}
+    for i, (name, t) in enumerate(tensors):
+        wide = t.dtype == torch.float64 or not t.is_floating_point()
+        out_dtype = torch.float64 if wide else torch.float32
+        n = t.numel()
+        k = min(n, left // (len(tensors) - i) // (8 if wide else 4))
+        flat = t.detach().reshape(-1)
+        entry = {"shape": list(t.shape), "dtype": str(t.dtype), "numel": n, "written": k}
+        if k < n:
+            idx = np.sort(np.random.default_rng(zlib.crc32(name.encode())).choice(n, size=k, replace=False))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+            entry["sample"] = "numpy.random.default_rng(zlib.crc32(name)).choice(numel, size=written, replace=False), sorted"
+        arr = flat.to(out_dtype).cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+        left -= arr.nbytes
+        manifest[name] = entry
+    with open(os.path.join(out_dir, "manifest.json"), "w") as f:
+        json.dump(manifest, f, indent=1)
+
+
+def measure_model(cx, model: str, steps: int, warmup: int, first_call: bool = False, roofline_only: bool = False,
+                  dump_dir: str | None = None):
     """value / e2e / roofline of one model, the procedure of the module docstring.
-    `roofline_only` (for ncu): one materialize, then 3 + steps launches of the dominant kernel's plan."""
+    `roofline_only` (for ncu): one materialize, then 3 + steps launches of the dominant kernel's plan.
+    `dump_dir`: where dump_outputs writes the model the timed `value` launches wrote into."""
     import torch
     import torch.distributed as dist
 
@@ -369,6 +409,8 @@ def measure_model(cx, model: str, steps: int, warmup: int, first_call: bool = Fa
             e1.record()
             barrier()
         res["ms"] = max_over_ranks(e0.elapsed_time(e1) / steps)
+        if dump_dir:
+            dump_outputs(keep, dump_dir if world == 1 else os.path.join(dump_dir, f"rank{rank}"))
     res["clk"] = clk.summary()
 
     # ---- roofline of the dominant kernel (most bytes), timed alone with the same events ----------
@@ -527,7 +569,7 @@ def run_ours(a):
 
     torch.manual_seed(1234)
     parallel.sync_rng(dev)  # the one collective: 16 bytes, rank 0 -> all
-    main = measure_model(cx, a.model, a.steps, a.warmup, first_call=True)
+    main = measure_model(cx, a.model, a.steps, a.warmup, first_call=True, dump_dir=a.dump_outputs)
 
     # ---- the other BASELINE configs, measured in the same run (smaller step counts) ----------------
     extra = {}
@@ -651,6 +693,9 @@ def main():
     ap.add_argument("--roofline-only", action="store_true",
                     help="for ncu: one materialize (1 launch per family), then 3+steps launches of the "
                          "dominant kernel's plan only; prints nothing")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the materialised model's parameters and buffers to DIR "
+                         "as <name>.npy (float32/float64, 64 MB at most; a fixed seeded sample of large tensors)")
     a = ap.parse_args()
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
     if a.impl == "reference":

@@ -11,6 +11,7 @@ import torch
 from torch import nn
 
 from oracle import cases
+from oracle import golden
 from torchdistx_b200.deferred_init import (deferred_init, is_deferred, last_materialize_stats, materialize_module,
                                            materialize_tensor)
 from torchdistx_b200.plan import InitPlan
@@ -121,12 +122,10 @@ def test_per_tensor_allocation_switch(tmp_path):
 
 # ---- partial writes through views ----------------------------------------------------------------
 @pytest.fixture(scope="module")
-def padded_reference(tmp_path_factory):
-    d = tmp_path_factory.mktemp("padref")
-    path = str(d / "p.pt")
-    subprocess.run([sys.executable, os.path.join(ROOT, "oracle", "ref_driver.py"), "--case", "padded_embeddings",
-                    "--dtype", "fp32", "--seed", "5", "--out", path], check=True, cwd=ROOT, timeout=300)
-    return torch.load(path)
+def padded_reference():
+    """The real reference, fp32, seed 5 (tests/golden/make_reference_outputs.py): per weight its padded
+    row and the `golden.summary` of the other rows."""
+    return golden.load("reference_gpu_cases")["padded_embeddings_fp32"]
 
 
 @pytest.mark.parametrize("dtype", ["fp32", "bf16"])
@@ -143,15 +142,15 @@ def test_padding_idx_embeddings_fuse_and_match_the_reference(dtype, padded_refer
     # the padded rows: bit-exact zeros (T0); everything else: the reference's distribution (T1)
     for name, row in (("torch_style", 3), ("hf_style", 0), ("last_row", 256)):
         w = getattr(m, name).weight.detach()
-        r = ref[f"{name}.weight"]
-        assert torch.equal(w[row].cpu(), torch.zeros_like(r[row], dtype=w.dtype)) and torch.equal(r[row], torch.zeros_like(r[row]))
+        r_row, rr = ref[f"{name}.weight"]["padded_row"], ref[f"{name}.weight"]["rest"]
+        assert torch.equal(w[row].cpu(), torch.zeros_like(r_row, dtype=w.dtype)) and torch.equal(r_row, torch.zeros_like(r_row))
         rest = torch.cat([w[:row], w[row + 1:]]).double().flatten()
-        rr = torch.cat([r[:row], r[row + 1:]]).double().flatten()
         n = rest.numel()
+        assert n == rr["numel"]
         assert (rest != 0).float().mean().item() > 0.99
         slack = 2.0 ** -8 if dtype == "bf16" else 0.0
-        assert abs(rest.mean().item() - rr.mean().item()) <= 5 * rr.std().item() / math.sqrt(n), name
-        assert abs(rest.std().item() / rr.std().item() - 1) <= 5 / math.sqrt(2 * n) + slack, name
+        assert abs(rest.mean().item() - rr["mean"]) <= 5 * rr["std"] / math.sqrt(n), name
+        assert abs(rest.std().item() / rr["std"] - 1) <= 5 / math.sqrt(2 * n) + slack, name
     h = m.halves.detach().float().cpu()
     assert torch.equal(h[32:], torch.full((32, 32), 0.5))
     assert abs(h[:16].std().item() / 0.2 - 1) < 0.15 and abs(h[16:32].std().item() / 0.1 - 1) < 0.15

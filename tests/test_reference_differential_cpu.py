@@ -1,6 +1,8 @@
-"""Differential run against the REAL reference (oracle/_ref) on random linked scripts, CPU device:
-both engines replay recorded ATen ops there, so every bit is comparable, random draws included
-(SURVEY.md 8c T0'); the eager run of the same script is the third opinion.
+"""Differential run against the REAL reference on random linked scripts, CPU device: both engines
+replay recorded ATen ops there, so every bit is comparable, random draws included (SURVEY.md 8c
+T0'); the eager run of the same script is the third opinion.  What the reference materialised
+(oracle/_ref, run on the same scripts by tests/golden/make_reference_outputs.py) is stored as
+`oracle.golden.value_digest`s: equal digests are what `same` below calls the same.
 
 What is asserted
   * there is no script on which the reference reproduces the eager construction and this engine
@@ -14,18 +16,14 @@ What is asserted
     is what nn.Embedding(padding_idx=...) does, is kept).  Eager PyTorch is the arbiter: the engine
     keeps the write.  On these scripts the reference matches eager far less often than the engine
     for that reason (printed, and asserted only as "not more often")."""
-import os
-import subprocess
-import sys
-
 import pytest
 import torch
 from torch import nn
 
 from oracle import fuzz_programs as P
+from oracle import golden
 from torchdistx_b200.deferred_init import deferred_init, materialize_module
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 N = 300
 
 
@@ -35,17 +33,15 @@ def same(x, y):
 
 
 @pytest.fixture(scope="module")
-def reference_runs(tmp_path_factory):
-    out = str(tmp_path_factory.mktemp("refdiff") / "ref.pt")
-    subprocess.run([sys.executable, os.path.join(ROOT, "oracle", "ref_fuzz_driver.py"), "--lo", "0", "--hi", str(N),
-                    "--out", out], check=True, cwd=ROOT, timeout=600)
-    return torch.load(out)
+def reference_runs():
+    return golden.load("reference_differential")
 
 
 def test_engine_is_never_wrong_where_the_reference_is_right(reference_runs):
     engine_eq_eager = ref_eq_eager = both = 0
+    assert len(reference_runs["scripts"]) == N
     for seed in range(N):
-        ref = reference_runs[seed]
+        ref = reference_runs["scripts"][seed]
         assert not isinstance(ref, str), (seed, ref)  # (the reference accepted every script)
         progs, links = P.differential_script(seed)
         m = deferred_init(P.LinkedHolder, progs, links)
@@ -57,9 +53,9 @@ def test_engine_is_never_wrong_where_the_reference_is_right(reference_runs):
         want = {k: v.detach() for k, v in eager.named_parameters()}
         assert set(mine) == set(ref) == set(want)
         e_ok = all(same(mine[k], want[k]) for k in want)
-        r_ok = all(same(ref[k], want[k]) for k in want)
+        r_ok = all(ref[k] == golden.value_digest(want[k]) for k in want)
         if r_ok:
-            assert all(same(mine[k], ref[k]) for k in ref), seed
+            assert all(golden.value_digest(mine[k]) == ref[k] for k in ref), seed
         engine_eq_eager += e_ok
         ref_eq_eager += r_ok
         both += e_ok and r_ok
@@ -67,7 +63,7 @@ def test_engine_is_never_wrong_where_the_reference_is_right(reference_runs):
     assert engine_eq_eager >= 0.95 * N and ref_eq_eager <= engine_eq_eager and both == ref_eq_eager
 
 
-def test_write_through_a_view_before_the_last_alias_is_kept():
+def test_write_through_a_view_before_the_last_alias_is_kept(reference_runs):
     def before():
         t = torch.ones(4, 4)
         t[1].zero_()
@@ -83,19 +79,8 @@ def test_write_through_a_view_before_the_last_alias_is_kept():
         m = deferred_init(fn)
         materialize_module(m)
         assert torch.equal(m[0].detach(), fn()[0].detach()), fn.__name__
-    # the reference, same two programs (a subprocess: it owns the same dispatch keys)
-    code = ("import sys, torch; sys.path.insert(0, %r)\n"
-            "from torch import nn\n"
-            "from oracle import ref_torchdistx as R\n"
-            "def before():\n"
-            "    t = torch.ones(4, 4); t[1].zero_(); return nn.ParameterList([nn.Parameter(t)])\n"
-            "def after():\n"
-            "    t = nn.Parameter(torch.ones(4, 4))\n"
-            "    with torch.no_grad(): t[1].zero_()\n"
-            "    return nn.ParameterList([t])\n"
-            "for fn in (before, after):\n"
-            "    m = R.deferred_init(fn); R.materialize_module(m); print(fn.__name__, m[0].detach()[1].tolist())\n" % ROOT)
-    out = subprocess.run([sys.executable, "-c", code], check=True, capture_output=True, text=True, cwd=ROOT, timeout=300).stdout
+    # the reference, same two programs: row 1 of what it materialised (make_reference_outputs.VIEW_WRITE)
+    out = reference_runs["view_write"]
     assert "after [0.0, 0.0, 0.0, 0.0]" in out, out
     # (if a later reference build keeps the write, this line is what changes -- and the docstring above)
     assert "before [1.0, 1.0, 1.0, 1.0]" in out, out

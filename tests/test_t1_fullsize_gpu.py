@@ -1,8 +1,8 @@
 """T1 parity at BASELINE tensor sizes (SURVEY.md section 8c, verbatim tolerances).
 
 The engine's CUDA output is compared with the REAL reference (oracle/_ref = pytorch/torchdistx
-compiled from its own sources, CPU device, subprocess) running the same program under the same
-seed, on
+compiled from its own sources, CPU device) running the same program under the same seed -- stored
+in tests/golden/reference_t1_fullsize.pt.gz by tests/golden/make_reference_outputs.py -- on
 
   * `llama8b_layer`      the 234,893,312-parameter sample of Llama-3-8B that bench.py times the
                          reference on (every linear at its real size: 4096x4096, 1024x4096,
@@ -18,6 +18,7 @@ Per RNG tensor (N elements, sigma = the reference sample's std), SURVEY 8c T1:
     |std/std_ref - 1|   <= 5 / sqrt(2N)            (+ 2^-8 for 16-bit outputs: the rounding term)
     hard range          uniform in [from, to), trunc_normal_ in [a, b]   (through the API)
     two-sample KS on an evenly strided 2^20-element subsample, alpha = 1e-3
+                        (the reference's subsample rebuilt from its 4096 quantiles: oracle/golden.py)
     no NaN / Inf
 
 Both sides of every comparison are samples, so these bounds are 3.5 standard deviations of the
@@ -33,22 +34,19 @@ Deterministic tensors stay T0: norm weights bit-exact; the rotary `inv_freq` buf
 arithmetic through `pow`, replayed by ATen's CUDA kernels) to 4 ulp of the reference's CPU result.
 """
 import math
-import os
-import subprocess
-import sys
 
 import pytest
 import torch
 
 from oracle import cases
+from oracle import golden
 from torchdistx_b200.deferred_init import deferred_init, last_materialize_stats, materialize_module
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SEED = 11
+SEED = 11  # (the reference's seed: make_reference_outputs.T1_SEED)
 SUBSAMPLE = 1 << 20
 
-# (case, dtype the ENGINE builds in, dtype the REFERENCE runs in, --round-to)
+# (case, dtype the ENGINE builds in, dtype the REFERENCE runs in, --round-to): make_reference_outputs.T1_RUNS
 RUNS = {
     "llama_bf16": ("llama8b_layer", "bf16", "fp32", "bf16"),
     "llama_cast": ("llama8b_layer_cast", "fp32", "fp32", ""),
@@ -57,28 +55,9 @@ RUNS = {
 }
 
 
-def run_reference(tmp, key):
-    case, _, ref_dtype, round_to = RUNS[key]
-    path = os.path.join(tmp, f"{key}.pt")
-    cmd = [sys.executable, os.path.join(ROOT, "oracle", "ref_driver.py"), "--case", case, "--dtype", ref_dtype,
-           "--seed", str(SEED), "--stats", "--out", path]
-    if round_to:
-        cmd += ["--round-to", round_to]
-    subprocess.run(cmd, check=True, cwd=ROOT, timeout=300)
-    return torch.load(path)
-
-
 @pytest.fixture(scope="module")
-def reference(tmp_path_factory):
-    tmp = str(tmp_path_factory.mktemp("t1_fullsize"))
-    cache = {}
-
-    def get(key):
-        if key not in cache:
-            cache[key] = run_reference(tmp, key)
-        return cache[key]
-
-    return get
+def reference():
+    return golden.load("reference_t1_fullsize")
 
 
 def build(key):
@@ -99,7 +78,7 @@ def check_t1(name, x, ref, sixteen_bit):
     if isinstance(ref, dict):
         assert ref["finite"] and ref["numel"] == n and tuple(ref["shape"]) == tuple(x.shape), name
         r_mean, r_std, stride = ref["mean"], ref["std"], ref["stride"]
-        r_sample = ref["sample"].double().numpy()
+        r_sample = golden.expand(ref["quantiles"], SUBSAMPLE)
         x_sample = xd[: stride * SUBSAMPLE: stride].cpu().numpy()
     else:
         rd = ref.double().flatten()
@@ -117,7 +96,7 @@ def check_t1(name, x, ref, sixteen_bit):
 
 @pytest.mark.parametrize("key", ["llama_bf16", "llama_cast"])
 def test_llama3_8b_sample_against_reference(key, reference):
-    ref = reference(key)
+    ref = reference[key]
     m = build(key)
     st = last_materialize_stats()
     mine = dict(list(m.named_parameters()) + list(m.named_buffers()))
@@ -154,7 +133,7 @@ def test_llama3_8b_sample_against_reference(key, reference):
 
 @pytest.mark.parametrize("key", ["big_fp32", "big_bf16"])
 def test_single_2p24_tensors_against_reference(key, reference):
-    ref = reference(key)
+    ref = reference[key]
     m = build(key)
     sixteen = key.endswith("bf16")
     st = last_materialize_stats()

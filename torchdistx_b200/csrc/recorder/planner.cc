@@ -28,6 +28,7 @@
 #include <ATen/detail/CUDAHooksInterface.h>
 #include <c10/cuda/CUDAFunctions.h>
 #include <cuda_runtime_api.h>
+#include <torch/csrc/utils/device_lazy_init.h>
 
 #include "fake_tensor.h"
 #include "stack_walk.h"
@@ -2422,7 +2423,10 @@ PipelinedMaterialize::PipelinedMaterialize(const MaterializeOptions& opts) : st_
   st_->threaded = host_threads_enabled();
   st_->items.reserve(1024);
   if (st_->threaded) {
-    if (at::hasCUDA() && c10::cuda::device_count() > 0) {
+    // Counting devices starts the CUDA runtime, which a child forked afterwards cannot use: like
+    // torch.cuda, mark such children (is_device_in_bad_fork), where a CPU-only call skips CUDA.
+    torch::utils::register_fork_handler_for_device_init(at::kCUDA);
+    if (!torch::utils::is_device_in_bad_fork(at::kCUDA) && at::hasCUDA() && c10::cuda::device_count() > 0) {
       // Only devices this call can touch, and only if they are in use already: asking for another
       // device's stream, or sitting on a device the process never used, would create a CUDA context
       // there (a CPU-only materialise on a GPU machine must not start CUDA at all).
